@@ -12,6 +12,7 @@ outside the hot path: the step starts from synthetic FPN features.
 
   python bench.py --gpus N --steps K --warmup W            # this repo's sm_100a path
   python bench.py --impl reference --gpus N ...            # the CPU oracle port (the reference is not installable)
+  python bench.py ... --dump-outputs DIR                   # also write the last timed step's outputs as DIR/<name>.npy
 
 N > 1 (torchrun): data-parallel frames exactly like the reference's DDP evaluation -- rank r lifts and renders
 its own frame -- plus the north-star's single all_gather of the rendered maps; per-GPU work is fixed (weak scaling).
@@ -35,6 +36,8 @@ WORKLOADS = {
     'nuscenes_depth_450x800': dict(ray_number=(450, 800), ray_img_size=(900, 1600), fpn_hw=(896, 1600)),
     'tiny': dict(ray_number=(32, 32), ray_img_size=(900, 1600), fpn_hw=(128, 256)),
 }
+# rays kept by --dump-outputs: 11 floats per ray over all outputs (depth, max-depth, acc, normal, rgb, pixel) = 46 MB
+DUMP_RAYS = 1 << 20
 
 
 def parse():
@@ -56,7 +59,15 @@ def parse():
     ap.add_argument('--no-strong', action='store_true', help='skip the strong-scaling (one frame sharded over the ranks) measurement')
     ap.add_argument('--scaling', default='weak', choices=['weak', 'strong'], help='which measurement is the headline `value`')
     ap.add_argument('--no-reference-gpu', action='store_true', help='skip the reference-style eager-PyTorch-on-GPU side figure')
-    return ap.parse_args()
+    ap.add_argument('--dump-outputs', metavar='DIR',
+                    help='after the timed steps, write what the timed step returned in its last step to DIR/<name>.npy '
+                         '(float32; a fixed, seeded sample of rays when the frame has more than %d)' % DUMP_RAYS)
+    a = ap.parse_args()
+    if a.steps < 1:
+        ap.error('--steps must be >= 1')
+    if a.dump_outputs and a.impl != 'b200':
+        ap.error('--dump-outputs needs --impl b200')
+    return a
 
 
 # ------------------------------------------------------------------------------------------ synthetic frame
@@ -91,6 +102,24 @@ def build_model(workload, device, color_dims=3):
             p.mul_(0.1)
         model.head.model.field.deviation_network.variance.fill_(0.3)
     return model.eval().to(device), cfg
+
+
+def dump_outputs(out, path):
+    """NeuSHead.render's return value as path/<key>.npy (float32): one row per (camera, ray) in the frame's flat order, and
+    ms_rays, the pixel table every camera shares, as each row's pixel.  A frame of more than DUMP_RAYS rays keeps the same
+    seeded sample of DUMP_RAYS rows in every array, so that the dumps of two runs with the same arguments line up.  With the
+    random background, ms_colors also depends on how many draws torch's CUDA generator made before the last step, which
+    --steps and --warmup change."""
+    import numpy as np
+    total = out['ms_depths'][0].numel()
+    n_pix = out['ms_rays'].shape[0]
+    idx = torch.arange(total)
+    if total > DUMP_RAYS:
+        idx = torch.randperm(total, generator=torch.Generator().manual_seed(0))[:DUMP_RAYS].sort().values
+    os.makedirs(path, exist_ok=True)
+    for k, v in out.items():
+        t, rows = (v, idx % n_pix) if k == 'ms_rays' else (v[0].reshape(total, *v[0].shape[3:]), idx)
+        np.save(os.path.join(path, k + '.npy'), t[rows.to(t.device)].float().cpu().numpy())
 
 
 # ------------------------------------------------------------------------------------------ clocks
@@ -242,7 +271,12 @@ def run_b200(args):
     K, W = args.steps, max(args.warmup, 3)
     _lib.profile_enable(True)
     sampler = ClockSampler(local) if rank == 0 else None
-    total_ms, launches, clocks = timed(lambda: gather(step(feats_d, metas_d)), K, W, sampler, sample_clocks=True,
+    last = {}                                          # what the timed step returned last (--dump-outputs)
+
+    def step_eager():
+        last['out'] = step(feats_d, metas_d)
+        return gather(last['out'])
+    total_ms, launches, clocks = timed(step_eager, K, W, sampler, sample_clocks=True,
                                        finalize=gather_join if world > 1 else None)
     prof = _lib.profile_read()
     ms_per_step_eager = total_ms / K
@@ -277,11 +311,14 @@ def run_b200(args):
                 graph.replay()
                 return gather(g_out)
             total_ms, _, _ = timed(step_graph, K, W, finalize=gather_join if world > 1 else None)
+            last['out'] = g_out
             issue = 'CUDA graph replay of the step (collective outside the graph)'
         else:
             issue = 'eager issue (graph capture failed: %s)' % why
     ms_per_step = total_ms / K
     value = world * rays_per_frame / (ms_per_step * 1e-3)
+    if args.dump_outputs and rank == 0:              # before anything below replays the graph into g_out again
+        dump_outputs(last['out'], args.dump_outputs)
 
     # ---- strong scaling of ONE frame (SURVEY 8e): query-sharded lifting (one all_gather of the planes per layer), slab-sharded
     # decode, ray-sharded render, one final all_gather -- selfocc_b200/dist.py.  Total work is fixed as N grows.
@@ -767,7 +804,7 @@ def run_reference(args):
         return                                     # rank 0 alone runs the CPU arm
     K, W = args.steps, args.warmup
     t0 = time.perf_counter()
-    cb = cpu_reference(args.workload, steps=max(min(K, 5), 3), warmup=min(W, 1), color_dims=args.color_dims)
+    cb = cpu_reference(args.workload, steps=K, warmup=min(W, 1), color_dims=args.color_dims)
     w = WORKLOADS[args.workload]
     line = {'metric': 'rendered rays/sec (6-cam 900x1600)', 'value': cb['value'], 'unit': 'rays/s', 'n_gpus': args.gpus,
             'steps': K, 'warmup': W, 'ms_per_step': cb['ms_per_step_extrapolated'], 'higher_is_better': True, 'scaling': 'weak',

@@ -32,7 +32,9 @@ def test_library_exports_every_declared_symbol():
 def test_sm100a_only():
     from selfocc_b200 import _lib, build
     build.build()
-    out = subprocess.run(['cuobjdump', '--list-elf', _lib.LIB_PATH], capture_output=True, text=True).stdout
+    nvcc = build._nvcc()      # the toolkit that built the library; its bin/ need not be on PATH
+    cuobjdump = os.path.join(os.path.dirname(nvcc), 'cuobjdump') if os.path.isabs(nvcc) else 'cuobjdump'
+    out = subprocess.run([cuobjdump, '--list-elf', _lib.LIB_PATH], capture_output=True, text=True).stdout
     archs = set(re.findall(r'sm_\d+a?', out))
     assert archs == {'sm_100a'}, archs
 
