@@ -28,7 +28,8 @@ extern "C" {
 #define SO_ERR_CUDA (-3)          /* a CUDA runtime call or launch failed; see so_last_cuda_error */
 #define SO_ERR_NO_DEVICE (-4)
 
-#define SO_ABI_VERSION 3   /* 2: so_render_train_forward gained pair_workspace; 3: packed render volume entry points */
+#define SO_ABI_VERSION 4   /* 2: so_render_train_forward gained pair_workspace; 3: packed render volume entry points;
+                              4: occupancy evaluation entry points */
 
 /* ABI version of the loaded library (compare with SO_ABI_VERSION). */
 int so_abi_version(void);
@@ -245,6 +246,41 @@ int so_depth_metric_sums(const float* sampled, const float* depth_gt, const uint
  * sdf [n], grad [n,3] (NULL ok), feat [n, n_feat] raw decoded channels 1.. (NULL ok). */
 int so_field_query(const float* vol_sdf, const float* vol_feat, const so_volume_desc* vol_host,
                    const float* points, int64_t n, float* sdf, float* grad, float* feat, void* stream);
+
+/* ---------------------------------------------------------------------------------------
+ * Occupancy evaluation (eval_iou.py:206-258, eval_iou_kitti.py:167-196).
+ *
+ * so_occ_classify: decoded volume -> uint8 labels per output voxel, without storing the get_uniform_sdf lattice
+ * (neus_head.py:265-293).  The lattice is [H = ny, W = nx, D = nz] with node (h, w, d) at metres (xs[w], ys[h], zs[d]);
+ * xs / ys / zs are the caller's torch.linspace vectors, and a node's value is exactly what so_field_query returns there.
+ *   points == NULL  lattice mode: the output grid IS the lattice (grid->n0 = ny, n1 = nx, n2 = nz).
+ *   points [n, 3]   resample mode (Occ3D): normalised (x, y, z) in [0, 1] (eval_iou.py:211-218); each output voxel is
+ *                   F.grid_sample(lattice, points[..., [2, 0, 1]] * 2 - 1, bilinear, align_corners=True, zeros padding).
+ * occ [n] = sdf <= thresh, then zeroed outside third-axis [z_lo, z_hi) and in the border rows (first axis: the first
+ * border[0] and last border[1] indices, second axis: border[2] / border[3]).
+ * sem [n] (NULL = not computed) = occ * lut[argmax_c logit_c], logits = vol_feat channels 3.. (h[..., 4:] of the
+ * lattice), first maximum; lut [lut_len >= n_feat - 3] uint8 (NULL = identity).  Logits are only gathered where occ is
+ * 1.  n_feat - 3 <= 32.  n = n0 * n1 * n2 voxels, row-major.
+ *
+ * so_occ_hist: hist[g * P + min(pred, P - 1)] += 1 for every i < n with mask[i] != 0 (mask NULL = all), g = gt[i];
+ * hist int64 [256, P], zero-filled by the caller and ACCUMULATED (across frames).  1 <= P <= SO_OCC_HIST_MAX_P.
+ * Integer counts: deterministic.  Every reference occupancy metric (MeanIoU, IoU, SSCMetrics) is a function of it.
+ */
+#define SO_OCC_HIST_MAX_P 32
+
+typedef struct so_occ_grid {
+  int32_t n0, n1, n2;     /* output grid shape */
+  int32_t z_lo, z_hi;     /* kept third-axis index range [z_lo, z_hi) */
+  int32_t border[4];      /* zeroed rows: first axis low, high; second axis low, high (>= 0) */
+  float thresh;           /* occupied: sdf <= thresh */
+} so_occ_grid;
+
+int so_occ_classify(const float* vol_sdf, const float* vol_feat, const so_volume_desc* vol_host, const float* xs,
+                    const float* ys, const float* zs, int32_t nx, int32_t ny, int32_t nz, const float* points,
+                    const so_occ_grid* grid_host, const uint8_t* lut, int32_t lut_len, uint8_t* occ, uint8_t* sem,
+                    void* stream);
+int so_occ_hist(const uint8_t* pred, const uint8_t* gt, const uint8_t* mask, int64_t n, int32_t P, int64_t* hist,
+                void* stream);
 
 /* ---------------------------------------------------------------------------------------
  * A7/A8  multi-scale deformable attention forward.  Drop-in for

@@ -8,7 +8,7 @@ import os
 
 _PKG = os.path.dirname(os.path.abspath(__file__))
 LIB_PATH = os.environ.get('SELFOCC_B200_LIB') or os.path.join(_PKG, 'lib', 'libselfocc_b200.so')   # env: experimental variant
-ABI_VERSION = 3
+ABI_VERSION = 4
 
 
 class AxisMap(C.Structure):
@@ -25,6 +25,11 @@ class RayDesc(C.Structure):
     _fields_ = [('n_cam', C.c_int32), ('rays_per_cam', C.c_int32), ('nx', C.c_int32), ('ny', C.c_int32),
                 ('sx', C.c_float), ('ox', C.c_float), ('sy', C.c_float), ('oy', C.c_float),
                 ('ray_begin', C.c_int64), ('ray_count', C.c_int64), ('chunk_len', C.c_int64)]
+
+
+class OccGrid(C.Structure):
+    _fields_ = [('n0', C.c_int32), ('n1', C.c_int32), ('n2', C.c_int32), ('z_lo', C.c_int32), ('z_hi', C.c_int32),
+                ('border', C.c_int32 * 4), ('thresh', C.c_float)]
 
 
 class RenderParams(C.Structure):
@@ -73,6 +78,9 @@ SIGNATURES = {
     'so_depth_metric_sample': (C.c_int, [_P, _P, _I, _I, _I, _I, _P, _P]),
     'so_depth_metric_sums': (C.c_int, [_P, _P, _P, _P, _I, _I, _P, _P]),
     'so_field_query': (C.c_int, [_P, _P, C.POINTER(VolumeDesc), _P, _L, _P, _P, _P, _P]),
+    'so_occ_classify': (C.c_int, [_P, _P, C.POINTER(VolumeDesc), _P, _P, _P, _I, _I, _I, _P, C.POINTER(OccGrid), _P, _I, _P, _P,
+                                  _P]),
+    'so_occ_hist': (C.c_int, [_P, _P, _P, _L, _I, _P, _P]),
     'so_msda_forward': (C.c_int, [_P, _P, _P, _P, _P, _P, _I, _I, _I, _I, _I, _I, _I, _P]),
     'so_msda_backward': (C.c_int, [_P, _P, _P, _P, _P, _P, _P, _P, _P, _I, _I, _I, _I, _I, _I, _I, _P]),
     'so_linear_force_ss': (C.c_int, [C.c_int]),

@@ -7,9 +7,11 @@ PKG = os.path.dirname(os.path.abspath(__file__))
 CSRC = os.path.join(PKG, 'csrc')
 LIB_DIR = os.path.join(PKG, 'lib')
 LIB = os.path.join(LIB_DIR, 'libselfocc_b200.so')
-SOURCES = ['abi.cu', 'render.cu', 'render_fast.cu', 'field_hess.cu', 'metric.cu', 'render_train.cu', 'decode.cu', 'msda.cu', 'gemm.cu', 'norm.cu']
+SOURCES = ['abi.cu', 'render.cu', 'render_fast.cu', 'field_hess.cu', 'metric.cu', 'occupancy.cu', 'render_train.cu', 'decode.cu', 'msda.cu', 'gemm.cu', 'norm.cu']
 # approx-unit math (ex2/rcp/rsq) without the denormal range-scaling wrappers: ~20 instructions per render sample
-PER_SOURCE_FLAGS = {'render.cu': ['-ftz=true'], 'render_fast.cu': ['-ftz=true'], 'render_train.cu': ['-ftz=true'], 'msda.cu': ['-ftz=true'], 'decode.cu': ['-ftz=true']}
+PER_SOURCE_FLAGS = {'render.cu': ['-ftz=true'], 'render_fast.cu': ['-ftz=true'], 'render_train.cu': ['-ftz=true'],
+                    'occupancy.cu': ['-ftz=true'],   # same field-query arithmetic as so_field_query (render.cu)
+                    'msda.cu': ['-ftz=true'], 'decode.cu': ['-ftz=true']}
 NVCC_FLAGS = ['-gencode', 'arch=compute_100a,code=sm_100a', '-O3', '-lineinfo', '-std=c++17',
               '--expt-relaxed-constexpr', '-Xcompiler', '-fPIC', '-Xptxas', '-v']
 

@@ -258,8 +258,7 @@ __global__ void __launch_bounds__(256) field_query_kernel(VolumeDev V, const flo
   if (i >= n) return;
   float x = pts[3 * i], y = pts[3 * i + 1], z = pts[3 * i + 2];
   float kh, kw, kd;
-  float gh = axis_m2g(V.ax[0], y, kh), gw = axis_m2g(V.ax[1], x, kw), gd = axis_m2g(V.ax[2], z, kd);
-  Taps t = make_taps(V, gh, gw, gd);
+  Taps t = field_taps(V, x, y, z, kh, kw, kd);
   float sdf, dgh, dgw, dgd;
   gather_sdf(V, t, sdf, dgh, dgw, dgd);
   if (sdf_out) sdf_out[i] = sdf;

@@ -131,6 +131,12 @@ __device__ __forceinline__ void gather_sdf(const VolumeDev& v, const Taps& t, fl
   dgd = fmaf(t.fh, dz1 - dz0, dz0);
 }
 
+// tap set of the field query at one point in metres (so_field_query; the occupancy lattice nodes of occupancy.cu)
+__device__ __forceinline__ Taps field_taps(const VolumeDev& V, float x, float y, float z, float& kh, float& kw, float& kd) {
+  float gh = axis_m2g(V.ax[0], y, kh), gw = axis_m2g(V.ax[1], x, kw), gd = axis_m2g(V.ax[2], z, kd);
+  return make_taps(V, gh, gw, gd);
+}
+
 // interior fast path: all 8 corners inside the volume (true for every sample strictly inside the AABB)
 __device__ __forceinline__ void gather_sdf_interior(const VolumeDev& v, int h0, int w0, int z0, float fh, float fw,
                                                     float fz, float& s, float& dgh, float& dgw, float& dgd) {

@@ -423,6 +423,47 @@ class NeuSHead(nn.Module):
         sdf, xyz = self.get_uniform_sdf(aabb, reso, device=device)
         return {'sdf': sdf, 'rep': representation, 'xyz': xyz}
 
+    @torch.no_grad()
+    def occupancy(self, aabb=None, resolution=None, thresh=0., points=None, sem_lut=None, z_keep=None, border=None):
+        """Occupancy / semantic labels of the prepared frame (eval_iou.py:206-258, eval_iou_kitti.py:167-196) in one
+        launch, without the get_uniform_sdf lattice of ``forward_occ``.  Returns {'occ': uint8} plus 'sem' (uint8) when
+        the head was built with ``return_sem``, shaped like the [H(y), W(x), D(z)] lattice of ``get_uniform_sdf(aabb,
+        resolution)`` or, when ``points`` ([n0, n1, n2, 3] normalised (x, y, z), e.g. occupancy.occ3d_points) is given,
+        like ``points[..., 0]``: the lattice trilinearly resampled there as F.grid_sample(align_corners=True) does.
+        occ = sdf <= thresh, zeroed outside third-axis ``z_keep = (lo, hi)`` (hi < 0 counts from the end, like a slice)
+        and in the ``border = (first lo, first hi, second lo, second hi)`` rows; sem = occ * sem_lut[argmax of the
+        semantic logits] (sem_lut None: the raw argmax).  Enqueues without synchronising once a list ``sem_lut`` has
+        been seen (its device copy is cached)."""
+        f = self.model.field
+        if f.vol_sdf is None:
+            raise RuntimeError('occupancy() called before prepare(): no decoded volume')
+        if sem_lut is not None and not self.return_sem:
+            raise ValueError('sem_lut needs a head built with return_sem=True')
+        dev = f.vol_sdf.device
+        aabb = self.aabb if aabb is None else aabb
+        resolution = self.resolution if resolution is None else resolution
+        # the node coordinates of get_uniform_sdf, computed the same way (neus_head.py:266-268)
+        xs = torch.linspace(aabb[0], aabb[3], int((aabb[3] - aabb[0]) / resolution), device=dev)
+        ys = torch.linspace(aabb[1], aabb[4], int((aabb[4] - aabb[1]) / resolution), device=dev)
+        zs = torch.linspace(aabb[2], aabb[5], int((aabb[5] - aabb[2]) / resolution), device=dev)
+        n2 = zs.numel() if points is None else points.shape[-2]
+        if z_keep is not None:
+            lo, hi = z_keep
+            z_keep = (lo, n2 + hi if hi < 0 else hi)
+        lut = None
+        if sem_lut is not None:
+            if torch.is_tensor(sem_lut):
+                lut = sem_lut.to(device=dev, dtype=torch.uint8).contiguous()
+            else:
+                key = (tuple(int(v) for v in sem_lut), dev)
+                if getattr(self, '_lut_cache', (None,))[0] != key:
+                    self._lut_cache = (key, torch.tensor(key[0], dtype=torch.uint8, device=dev))
+                lut = self._lut_cache[1]
+        pts = None if points is None else points.to(device=dev, dtype=torch.float32).contiguous()
+        occ, sem = ops.occ_classify(f.vol_sdf, f.vol_feat, f.desc, xs, ys, zs, points=pts, thresh=thresh, z_keep=z_keep,
+                                    border=border, lut=lut, want_sem=self.return_sem)
+        return {'occ': occ, 'sem': sem} if self.return_sem else {'occ': occ}
+
     def forward(self, representation, metas=None, **kwargs):
         """neus_head.py:473-713 (training form: per-sample weights / ts / deltas / eik_grad)."""
         if self.return_second_grad and not self.second_grad_assumption:

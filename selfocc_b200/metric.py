@@ -4,6 +4,8 @@
 (``so_depth_metric_sample`` + ``so_depth_metric_sums``) and a sort-based masked median, so a frame's metric step
 enqueues without synchronising."""
 import ctypes as C
+import logging
+import numpy as np
 import torch
 import torch.nn as nn
 
@@ -100,3 +102,169 @@ class DepthMetric(nn.Module):
                     logger.info('%12s | ' % name + ' '.join('%s %.3f' % (k, res[k][ti, cam]) for k in KEYS + ('scaling',)))
                 logger.info('%12s | ' % 'All' + ' '.join('%s %.3f' % (k, res[k][ti].mean()) for k in KEYS + ('scaling',)))
         return res
+
+
+# --------------------------------------------------------------------------------------- occupancy metrics
+# utils/metric_util.py:66-244 and utils/scenerf_metric.py.  The reference accumulates per-class float32 counters with a
+# host sync per class per frame (.item() / .tolist()); every one of its numbers is a function of the joint (gt, pred)
+# label histogram, which so_occ_hist accumulates on the device as exact int64 counts without synchronising.  The float32
+# totals of the reference stop counting exactly once a total passes 2^24 voxels (a few dozen Occ3D frames for the
+# empty class); these counts do not, and the ratios are formed in float64.
+def _occ_labels(t):
+    return t.to(torch.uint8).contiguous().reshape(-1)
+
+
+class _OccHistogram:
+    """int64 hist[g, min(p, P - 1)] over uint8 labels; column P - 1 collects every prediction >= P - 1."""
+
+    P = 2
+
+    def reset(self):
+        self.hist = torch.zeros(256, self.P, dtype=torch.int64, device='cuda' if torch.cuda.is_available() else 'cpu')
+
+    def _accumulate(self, outputs, targets, mask=None):
+        from .ops import occ_hist
+        pred, gt = _occ_labels(outputs), _occ_labels(targets)
+        occ_hist(pred, gt, self.hist, None if mask is None else _occ_labels(mask))
+
+    def _reduced(self):
+        """The histogram summed over ranks (when torch.distributed is initialised), as a host int64 tensor."""
+        import torch.distributed as dist
+        h = self.hist
+        if dist.is_available() and dist.is_initialized():
+            h = h.clone()
+            dist.all_reduce(h)
+        return h.cpu()
+
+
+def _ratio(a, b):
+    return a / b if b else float('nan')
+
+
+class MeanIoU(_OccHistogram):
+    """Per-class IoU + non-empty IoU (utils/metric_util.py:66-165): same constructor, ``reset / _after_step /
+    _after_epoch``.  Labels are integers in [0, 255]; outputs outside [0, max(class_indices, empty_label)] count as
+    "some other non-empty class", as in the reference.  The dict-target branch (metric_util.py:93-105) is not
+    provided: no reference script uses it."""
+
+    def __init__(self, class_indices, empty_label, label_str, use_mask=False, dataset_empty_label=17, name='none'):
+        self.class_indices = list(class_indices)
+        self.num_classes = len(self.class_indices)
+        self.empty_label, self.dataset_empty_label = empty_label, dataset_empty_label
+        self.label_str, self.use_mask, self.name = label_str, use_mask, name
+        self.P = max(self.class_indices + [empty_label]) + 2
+        if min(self.class_indices + [empty_label]) < 0 or self.P > 32:
+            raise ValueError('MeanIoU: class indices and the empty label must lie in [0, 30]')
+
+    @torch.no_grad()
+    def _after_step(self, outputs, targets, mask=None):
+        """outputs, targets: integer label volumes of one shape; mask: bool / 0-1 voxels to count (None = all)."""
+        if not torch.is_tensor(targets):
+            raise NotImplementedError('MeanIoU: the dict-target branch of the reference is not provided')
+        self._accumulate(outputs, targets, mask)
+
+    def counts(self):
+        """(total_seen, total_correct, total_positive) int lists of the reference, the last entry the non-empty row."""
+        h = self._reduced()
+        e = self.empty_label
+        seen = [int(h[c].sum()) for c in self.class_indices]
+        correct = [int(h[c, c]) for c in self.class_indices]
+        positive = [int(h[:, c].sum()) for c in self.class_indices]
+        total = int(h.sum())
+        ne = torch.ones(256, dtype=torch.bool)
+        ne[e] = False
+        ne_p = torch.ones(self.P, dtype=torch.bool)
+        ne_p[e] = False
+        seen.append(total - int(h[e].sum()))
+        correct.append(int(h[ne][:, ne_p].sum()))
+        positive.append(total - int(h[:, e].sum()))
+        return seen, correct, positive
+
+    def _after_epoch(self):
+        """(mIoU * 100, non-empty IoU * 100); a class never seen in the ground truth counts as IoU 1."""
+        seen, correct, positive = self.counts()
+        ious = [1.0 if seen[i] == 0 else _ratio(correct[i], seen[i] + positive[i] - correct[i]) for i in range(self.num_classes)]
+        miou = float(np.mean(ious))
+        log = logging.getLogger('selfocc_b200')
+        log.info('Validation per class iou %s:', self.name)
+        for i, s in enumerate(self.label_str):
+            prec = _ratio(correct[i], positive[i]) if positive[i] else 0.
+            rec = _ratio(correct[i], seen[i]) if seen[i] else 1.
+            log.info('%s : %.2f%%, %.2f, %.2f', s, ious[i] * 100, prec, rec)
+        occ_iou = _ratio(correct[-1], seen[-1] + positive[-1] - correct[-1])
+        return miou * 100, occ_iou * 100
+
+
+class IoU(_OccHistogram):
+    """Occupied-voxel IoU of eval_iou_kitti.py (utils/metric_util.py:168-244).  ``_after_step(outputs, targets)``:
+    outputs a 0/1 occupancy volume; targets either the raw label volume of the same shape (occupied = label not in
+    {0, 255}, no host sync) or, as in the reference, the [K, 3] coordinates of the occupied voxels."""
+
+    P = 2
+
+    def __init__(self, use_mask=False):
+        self.class_indices, self.num_classes, self.label_str, self.use_mask = [0], 1, ['occupied'], use_mask
+
+    @torch.no_grad()
+    def _after_step(self, outputs, targets, occ3d=False):
+        if occ3d:
+            raise NotImplementedError('IoU._after_step_occ3d is not provided: no reference script uses it')
+        if targets.shape != outputs.shape:
+            idx = targets.long()
+            occ = torch.zeros(outputs.shape, dtype=torch.uint8, device=outputs.device)
+            occ[tuple(idx.t())] = 1
+            targets = occ
+        self._accumulate(outputs, targets)
+
+    def counts(self):
+        h = self._reduced()
+        occ_rows = h[1:255]
+        return int(occ_rows.sum()), int(occ_rows[:, 1].sum()), int(h[:, 1].sum())
+
+    def _after_epoch(self):
+        """IoU * 100 of the occupied class (1 if no voxel is occupied in the ground truth)."""
+        seen, correct, positive = self.counts()
+        iou = 1.0 if seen == 0 else _ratio(correct, seen + positive - correct)
+        logging.getLogger('selfocc_b200').info('Final iou: %s', iou * 100)
+        return iou * 100
+
+
+class SSCMetrics(_OccHistogram):
+    """Scene-completion metrics of eval_iou_kitti.py (utils/scenerf_metric.py:39-215): ``reset / add_batch /
+    get_stats``.  Completion counts voxels with gt != 255 (occupied: label > 0); the per-class counts compare RAW labels
+    0 .. n_classes - 1, so SSCMetrics(2) fed SemanticKITTI labels scores "class 1" as gt == 1, as the reference does."""
+
+    def __init__(self, n_classes):
+        self.n_classes = n_classes
+        self.P = n_classes + 1
+        if not 1 <= n_classes <= 31:
+            raise ValueError('SSCMetrics: n_classes must lie in [1, 31]')
+        self.reset()
+
+    @torch.no_grad()
+    def add_batch(self, y_pred, y_true, nonempty=None, nonsurface=None):
+        if nonsurface is not None:
+            raise NotImplementedError('SSCMetrics: nonsurface is not provided (no reference script passes it)')
+        self._accumulate(y_pred, y_true, nonempty)
+
+    def counts(self):
+        """(completion tp, fp, fn, per-class tps, fps, fns) as ints."""
+        h = self._reduced()
+        h = torch.cat([h[:255], torch.zeros(1, self.P, dtype=h.dtype)])      # gt == 255 is ignored
+        occ_g = h[1:]
+        tp, fp, fn = int(occ_g[:, 1:].sum()), int(h[0, 1:].sum()), int(occ_g[:, 0].sum())
+        C = self.n_classes
+        tps = [int(h[j, j]) for j in range(C)]
+        fps = [int(h[:, j].sum()) - tps[j] for j in range(C)]
+        fns = [int(h[j].sum()) - tps[j] for j in range(C)]
+        return tp, fp, fn, tps, fps, fns
+
+    def get_stats(self):
+        tp, fp, fn, tps, fps, fns = self.counts()
+        if tp != 0:
+            precision, recall, iou = tp / (tp + fp), tp / (tp + fn), tp / (tp + fp + fn)
+        else:
+            precision, recall, iou = 0., 0., 0.
+        iou_ssc = torch.tensor([a / (a + b + c + 1e-5) for a, b, c in zip(tps, fps, fns)], dtype=torch.float64)
+        return {'precision': precision, 'recall': recall, 'iou': iou, 'iou_ssc': iou_ssc,
+                'iou_ssc_mean': float(iou_ssc[1:].mean())}

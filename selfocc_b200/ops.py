@@ -157,6 +157,44 @@ def field_query(vol_sdf, vol_feat, desc, points, want_grad=False, want_feat=Fals
     return sdf, grad, feat
 
 
+# --------------------------------------------------------------------------------------- occupancy evaluation
+def occ_classify(vol_sdf, vol_feat, desc, xs, ys, zs, points=None, thresh=0., z_keep=None, border=None, lut=None, want_sem=False):
+    """Decoded volume -> (occ u8, sem u8 | None) shaped like the [len(ys), len(xs), len(zs)] lattice (points None) or like
+    points[..., 0] (points [n0, n1, n2, 3] normalised (x, y, z), trilinear resample of the lattice).  z_keep = (lo, hi)
+    kept third-axis range (default all), border = (first lo, first hi, second lo, second hi) zeroed rows (default 0);
+    lut: uint8 table applied to the semantic argmax (None = raw argmax)."""
+    lib = _lib.load()
+    _chk(vol_sdf, name='vol_sdf'); _chk(vol_feat, name='vol_feat')
+    _chk(xs, name='xs'); _chk(ys, name='ys'); _chk(zs, name='zs'); _chk(points, name='points'); _chk(lut, torch.uint8, 'lut')
+    shape = (ys.numel(), xs.numel(), zs.numel()) if points is None else tuple(points.shape[:-1])
+    if len(shape) != 3 or (points is not None and points.shape[-1] != 3):
+        raise ValueError('points must be [n0, n1, n2, 3], got %s' % (tuple(points.shape),))
+    g = _lib.OccGrid()
+    g.n0, g.n1, g.n2 = shape
+    g.z_lo, g.z_hi = (0, shape[2]) if z_keep is None else (int(z_keep[0]), int(z_keep[1]))
+    for i, b in enumerate((0, 0, 0, 0) if border is None else border):
+        g.border[i] = int(b)
+    g.thresh = float(thresh)
+    occ = torch.empty(shape, device=vol_sdf.device, dtype=torch.uint8)
+    sem = torch.empty(shape, device=vol_sdf.device, dtype=torch.uint8) if want_sem else None
+    _lib.check(lib.so_occ_classify(_p(vol_sdf), _p(vol_feat), C.byref(desc), _p(xs), _p(ys), _p(zs), xs.numel(), ys.numel(),
+                                   zs.numel(), _p(points), C.byref(g), _p(lut), 0 if lut is None else lut.numel(), _p(occ), _p(sem),
+                                   _stream()), 'so_occ_classify')
+    return occ, sem
+
+
+def occ_hist(pred, gt, hist, mask=None):
+    """hist int64 [256, P] += joint (gt, min(pred, P - 1)) counts over the voxels where mask != 0; pred, gt, mask uint8."""
+    lib = _lib.load()
+    _chk(pred, torch.uint8, 'pred'); _chk(gt, torch.uint8, 'gt'); _chk(mask, torch.uint8, 'mask'); _chk(hist, torch.int64, 'hist')
+    n = pred.numel()
+    if gt.numel() != n or (mask is not None and mask.numel() != n) or hist.dim() != 2 or hist.shape[0] != 256:
+        raise ValueError('occ_hist: pred %s, gt %s, mask %s, hist %s' % (tuple(pred.shape), tuple(gt.shape),
+                                                                        None if mask is None else tuple(mask.shape), tuple(hist.shape)))
+    _lib.check(lib.so_occ_hist(_p(pred), _p(gt), _p(mask), n, hist.shape[1], _p(hist), _stream()), 'so_occ_hist')
+    return hist
+
+
 # --------------------------------------------------------------------------------------- A4-A8
 def msda_forward(value, spatial_shapes, level_start_index, loc, weights):
     lib = _lib.load()
