@@ -28,8 +28,8 @@ extern "C" {
 #define SO_ERR_CUDA (-3)          /* a CUDA runtime call or launch failed; see so_last_cuda_error */
 #define SO_ERR_NO_DEVICE (-4)
 
-#define SO_ABI_VERSION 4   /* 2: so_render_train_forward gained pair_workspace; 3: packed render volume entry points;
-                              4: occupancy evaluation entry points */
+#define SO_ABI_VERSION 5   /* 2: so_render_train_forward gained pair_workspace; 3: packed render volume entry points;
+                              4: occupancy evaluation entry points; 5: reprojection loss entry points */
 
 /* ABI version of the loaded library (compare with SO_ABI_VERSION). */
 int so_abi_version(void);
@@ -281,6 +281,42 @@ int so_occ_classify(const float* vol_sdf, const float* vol_feat, const so_volume
                     void* stream);
 int so_occ_hist(const uint8_t* pred, const uint8_t* gt, const uint8_t* mask, int64_t n, int32_t P, int64_t* hist,
                 void* stream);
+
+/* ---------------------------------------------------------------------------------------
+ * Self-supervised reprojection loss (loss/reproj_loss_mono_multi_new_combine.py:108-245, variant SO_REPROJ_COMBINE;
+ * loss/reproj_loss_mono_multi_new.py:117-288, variant SO_REPROJ_MONO_MULTI_NEW, sdf_loss=False).
+ *
+ * Inputs are the training head's per-sample outputs in its ray layout: N cameras x R rays x S CONTIGUOUS samples,
+ * rays in order (ray_indices[cam] = arange(R).repeat_interleave(S); so_reproj_check_layout verifies that).
+ *   curr, prev, next [N, 3, img_h, img_w]   pix [R, 2] pixel (x, y) = ms_rays   img2prev, img2next [N, 4, 4]
+ *   weights, ts [N, R * S]   deltas [N, R * S] or NULL (w <- delta < eps ? 0 : w / max(delta, eps))
+ * so_reproj_forward writes loss[0] = the reference's return value (mean over rays, then over cameras; the caller applies
+ * the loss weight) and keeps in `workspace` what the backward needs; so_reproj_backward takes the device scalar
+ * g_loss[0] = d total / d loss and the SAME inputs and workspace, and writes g_weights [N, R * S] (no gradient w.r.t. ts,
+ * deltas, images or transforms).  Combine samples the images with padding_mode='border', MonoMultiNew with zeros.
+ * ssim != 0 needs grid_h * grid_w == R (ray_resize), grid_h, grid_w >= 2.  Deterministic: no atomics.
+ * so_reproj_workspace_floats: floats of workspace for `desc` (-1: invalid desc). */
+#define SO_REPROJ_COMBINE 0
+#define SO_REPROJ_MONO_MULTI_NEW 1
+
+typedef struct so_reproj_desc {
+  int32_t variant;                     /* SO_REPROJ_* */
+  int32_t n_cam, n_rays, n_samples;    /* N, R, S */
+  int32_t img_h, img_w;                /* image tensor size */
+  float size_h, size_w;                /* img_size the pixel coordinates are normalised by */
+  int32_t grid_h, grid_w;              /* ray_resize, read iff ssim */
+  int32_t ssim, automask;              /* !no_ssim, !no_automask */
+} so_reproj_desc;
+
+int64_t so_reproj_workspace_floats(const so_reproj_desc* desc_host);
+int so_reproj_forward(const so_reproj_desc* desc_host, const float* curr, const float* prev, const float* next,
+                      const float* pix, const float* img2prev, const float* img2next, const float* weights, const float* ts,
+                      const float* deltas, float* loss, float* workspace, void* stream);
+int so_reproj_backward(const so_reproj_desc* desc_host, const float* curr, const float* prev, const float* next,
+                       const float* pix, const float* img2prev, const float* img2next, const float* weights, const float* ts,
+                       const float* deltas, const float* g_loss, float* g_weights, float* workspace, void* stream);
+/* bad[0] |= 1 if ray_idx[i] != i / n_samples for some i < n (bad zero-filled by the caller; no synchronisation). */
+int so_reproj_check_layout(const int64_t* ray_idx, int64_t n, int32_t n_samples, int32_t* bad, void* stream);
 
 /* ---------------------------------------------------------------------------------------
  * A7/A8  multi-scale deformable attention forward.  Drop-in for

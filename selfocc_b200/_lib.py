@@ -8,7 +8,7 @@ import os
 
 _PKG = os.path.dirname(os.path.abspath(__file__))
 LIB_PATH = os.environ.get('SELFOCC_B200_LIB') or os.path.join(_PKG, 'lib', 'libselfocc_b200.so')   # env: experimental variant
-ABI_VERSION = 4
+ABI_VERSION = 5
 
 
 class AxisMap(C.Structure):
@@ -30,6 +30,15 @@ class RayDesc(C.Structure):
 class OccGrid(C.Structure):
     _fields_ = [('n0', C.c_int32), ('n1', C.c_int32), ('n2', C.c_int32), ('z_lo', C.c_int32), ('z_hi', C.c_int32),
                 ('border', C.c_int32 * 4), ('thresh', C.c_float)]
+
+
+class ReprojDesc(C.Structure):
+    _fields_ = [('variant', C.c_int32), ('n_cam', C.c_int32), ('n_rays', C.c_int32), ('n_samples', C.c_int32),
+                ('img_h', C.c_int32), ('img_w', C.c_int32), ('size_h', C.c_float), ('size_w', C.c_float),
+                ('grid_h', C.c_int32), ('grid_w', C.c_int32), ('ssim', C.c_int32), ('automask', C.c_int32)]
+
+
+REPROJ_COMBINE, REPROJ_MONO_MULTI_NEW = 0, 1
 
 
 class RenderParams(C.Structure):
@@ -81,6 +90,10 @@ SIGNATURES = {
     'so_occ_classify': (C.c_int, [_P, _P, C.POINTER(VolumeDesc), _P, _P, _P, _I, _I, _I, _P, C.POINTER(OccGrid), _P, _I, _P, _P,
                                   _P]),
     'so_occ_hist': (C.c_int, [_P, _P, _P, _L, _I, _P, _P]),
+    'so_reproj_workspace_floats': (_L, [C.POINTER(ReprojDesc)]),
+    'so_reproj_forward': (C.c_int, [C.POINTER(ReprojDesc)] + [_P] * 12),
+    'so_reproj_backward': (C.c_int, [C.POINTER(ReprojDesc)] + [_P] * 13),
+    'so_reproj_check_layout': (C.c_int, [_P, _L, _I, _P, _P]),
     'so_msda_forward': (C.c_int, [_P, _P, _P, _P, _P, _P, _I, _I, _I, _I, _I, _I, _I, _P]),
     'so_msda_backward': (C.c_int, [_P, _P, _P, _P, _P, _P, _P, _P, _P, _I, _I, _I, _I, _I, _I, _I, _P]),
     'so_linear_force_ss': (C.c_int, [C.c_int]),

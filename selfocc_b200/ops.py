@@ -659,3 +659,91 @@ def tpv_self_attn_forward_rows(value_rows, Hd, Dh, spatial_shapes, level_start_i
                                                     v.shape[0], Hd, Dh, Q, L, P, vld, old, lld, _stream()),
                'so_tpv_self_attn_forward_strided')
     return out
+
+
+# --------------------------------------------------------------------------------------- reprojection loss
+def make_reproj_desc(combine, n_cam, n_rays, n_samples, img_hw, img_size, ray_resize=None, ssim=True, automask=True):
+    """so_reproj_desc of one loss call; img_hw = the image tensor's (H, W), img_size = the (h, w) pixels are normalised by."""
+    d = _lib.ReprojDesc()
+    d.variant = _lib.REPROJ_COMBINE if combine else _lib.REPROJ_MONO_MULTI_NEW
+    d.n_cam, d.n_rays, d.n_samples = int(n_cam), int(n_rays), int(n_samples)
+    d.img_h, d.img_w = int(img_hw[0]), int(img_hw[1])
+    d.size_h, d.size_w = float(img_size[0]), float(img_size[1])
+    d.grid_h, d.grid_w = (int(ray_resize[0]), int(ray_resize[1])) if ray_resize is not None else (0, 0)
+    d.ssim, d.automask = int(bool(ssim)), int(bool(automask))
+    return d
+
+
+def _reproj_args(desc, curr, prev, nxt, pix, img2prev, img2next, weights, ts, deltas):
+    N, R, S = desc.n_cam, desc.n_rays, desc.n_samples
+    for n, t in (('curr', curr), ('prev', prev), ('next', nxt)):
+        if _chk(t, name=n).shape != (N, 3, desc.img_h, desc.img_w):
+            raise ValueError('%s must be [%d, 3, %d, %d], got %s' % (n, N, desc.img_h, desc.img_w, tuple(t.shape)))
+    for n, t, shp in (('pix', pix, (R, 2)), ('img2prev', img2prev, (N, 4, 4)), ('img2next', img2next, (N, 4, 4)),
+                      ('weights', weights, (N, R * S)), ('ts', ts, (N, R * S)), ('deltas', deltas, (N, R * S))):
+        if t is not None and tuple(_chk(t, name=n).shape) != shp:
+            raise ValueError('%s must be %s, got %s' % (n, shp, tuple(t.shape)))
+    return [_p(t) for t in (curr, prev, nxt, pix, img2prev, img2next, weights, ts, deltas)]
+
+
+def reproj_forward(desc, curr, prev, nxt, pix, img2prev, img2next, weights, ts, deltas=None):
+    """-> (loss [1] before the loss weight, workspace for reproj_backward).  Shapes as in so_reproj_forward."""
+    lib = _lib.load()
+    args = _reproj_args(desc, curr, prev, nxt, pix, img2prev, img2next, weights, ts, deltas)
+    nws = lib.so_reproj_workspace_floats(C.byref(desc))
+    if nws < 0:
+        raise ValueError('invalid reprojection loss configuration (ray_resize must tile the %d rays)' % desc.n_rays)
+    ws = torch.empty(nws, device=curr.device, dtype=torch.float32)
+    loss = torch.empty(1, device=curr.device, dtype=torch.float32)
+    _lib.check(lib.so_reproj_forward(C.byref(desc), *args, _p(loss), _p(ws), _stream()), 'so_reproj_forward')
+    return loss, ws
+
+
+def reproj_backward(desc, curr, prev, nxt, pix, img2prev, img2next, weights, ts, deltas, g_loss, ws):
+    """g_loss [1] (device) -> g_weights [N, R * S]; ws from the reproj_forward of the same inputs."""
+    lib = _lib.load()
+    args = _reproj_args(desc, curr, prev, nxt, pix, img2prev, img2next, weights, ts, deltas)
+    _chk(g_loss, name='g_loss'); _chk(ws, name='workspace')
+    g_w = torch.empty_like(weights)
+    _lib.check(lib.so_reproj_backward(C.byref(desc), *args, _p(g_loss), _p(g_w), _p(ws), _stream()), 'so_reproj_backward')
+    return g_w
+
+
+def reproj_workspace_views(desc, ws):
+    """Named views of a forward's workspace (test hook): counts [N, R, 2] of valid samples per ray (Combine: [.., 0] =
+    samples with either projection valid), proj [N, R] per-ray loss, choice [N, R] index of the min."""
+    N, R = desc.n_cam, desc.n_rays
+    nr = N * R
+    sums = ws[9 * nr:21 * nr].reshape(N, R, 12)
+    counts = sums[..., 5:6] if desc.variant == _lib.REPROJ_COMBINE else sums[..., 10:12]
+    return dict(counts=counts, proj=ws[21 * nr:22 * nr].reshape(N, R), choice=ws[22 * nr:23 * nr].reshape(N, R))
+
+
+def reproj_check_layout(ray_idx, n_samples, bad):
+    """bad int32 [1] |= 1 unless ray_idx == arange(n / n_samples).repeat_interleave(n_samples); no synchronisation."""
+    lib = _lib.load()
+    _chk(ray_idx, torch.int64, 'ray_indices'); _chk(bad, torch.int32, 'bad')
+    _lib.check(lib.so_reproj_check_layout(_p(ray_idx), ray_idx.numel(), int(n_samples), _p(bad), _stream()),
+               'so_reproj_check_layout')
+
+
+class ReprojLossFunction(torch.autograd.Function):
+    """Reprojection loss, differentiable w.r.t. the stacked per-camera weights [N, R * S] only (ts, deltas, images and
+    transforms carry no gradient).  forward(weights, desc, curr, prev, next, pix, img2prev, img2next, ts, deltas) -> loss."""
+
+    @staticmethod
+    def forward(ctx, weights, desc, curr, prev, nxt, pix, img2prev, img2next, ts, deltas):
+        loss, ws = reproj_forward(desc, curr, prev, nxt, pix, img2prev, img2next, weights, ts, deltas)
+        ctx.desc = desc
+        ctx.save_for_backward(weights, curr, prev, nxt, pix, img2prev, img2next, ts,
+                              deltas if deltas is not None else weights.new_empty(0), ws)
+        ctx.has_deltas = deltas is not None
+        return loss.reshape(())
+
+    @staticmethod
+    @torch.autograd.function.once_differentiable
+    def backward(ctx, g):
+        weights, curr, prev, nxt, pix, img2prev, img2next, ts, deltas, ws = ctx.saved_tensors
+        g_w = reproj_backward(ctx.desc, curr, prev, nxt, pix, img2prev, img2next, weights, ts,
+                              deltas if ctx.has_deltas else None, g.reshape(1).contiguous(), ws)
+        return (g_w,) + (None,) * 9
